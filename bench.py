@@ -1,10 +1,15 @@
 #!/usr/bin/env python
 """bench.py -- Score() prompts/sec @4K tokens against a 10M-block / 256-pod index (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (GetPodScores steps 2-4, pkg/kvcache/indexer.go:141-163) over one
-batch of synthetic 4096-token prompts.
+batch of synthetic 4096-token prompts.  --steps sets the number of timed steps of `value`.
+
+--dump-outputs DIR writes what the last timed step returned to its caller, as .npy files: scores.npy (dense
+score rows, float64), has_keys.npy (float32) and prompt_index.npy (which prompts of the batch the rows belong to,
+float64).  Batches above 16 K prompts are sampled (fixed seed, 32 MiB of rows).  The inputs depend only on the
+arguments, so the files of two builds can be compared one to one.  Rank 0 writes its own batch.
 
   value     whole-job prompts/s with the batch already resident in HBM (kvidx_score_batch_dev)
   e2e       the same metric through the host-buffer C-ABI call (kvidx_score_batch): pinned host tokens
@@ -101,6 +106,24 @@ def device_queries(wl, q0, q1, device, full_depth=False, chunk=8192):
         mm = torch.from_numpy(m[c0:c1]).to(device)[:, None] * wl.B
         out[c0:c1] = torch.where(col < mm, dtok, tail).to(torch.int32)
     return out, doc, m
+
+
+DUMP_ROWS = 16384          # 16 K dense rows of 256 float64 scores = 32 MiB
+
+
+def dump_rows(n):
+    """Prompts of an n-prompt batch that --dump-outputs writes: all of them up to DUMP_ROWS, else a fixed seeded sample."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_outputs(out_dir, rows, scores, has_keys):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("prompt_index", rows.astype(np.float64)), ("scores", np.asarray(scores, np.float64)),
+                    ("has_keys", np.asarray(has_keys, np.float32))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log("[dump] %d score rows of the last timed step -> %s" % (len(rows), out_dir))
 
 
 def algorithmic_bytes(wl, m):
@@ -225,10 +248,13 @@ def run_reference(args):
         toks, doc, m = wl.queries(q, q + sample)
         q += sample
         off = np.arange(0, (sample + 1) * wl.T, wl.T, dtype=np.int64)
-        _, _, el, l = co.score_batch(toks.reshape(-1), off, n_threads=threads, want_scores=True, want_latency=True)
+        scores, has, el, l = co.score_batch(toks.reshape(-1), off, n_threads=threads, want_scores=True, want_latency=True)
         if step >= args.warmup:
             times.append(el)
             lat.append(l)
+    if args.dump_outputs:
+        rows = dump_rows(sample)
+        dump_outputs(args.dump_outputs, rows, scores[rows], has[rows])
     total = sum(times)
     value = sample * len(times) / total
     lat = np.concatenate(lat)
@@ -256,14 +282,17 @@ def go_probe():
     (fxamacker/cbor/v2 v2.7.0) are on this box, oracle/goprobe runs the reference's own hash call shape
     (token_processor.go:94-112) over tests/golden/hash_kats.json and the result is recorded; otherwise the reason is."""
     import shutil
+    import tempfile
     go = shutil.which("go")
     if not go:
         return {"go": None, "pinned": False, "why": "no go toolchain on this box"}
     try:
         ver = subprocess.run([go, "version"], capture_output=True, text=True, timeout=20).stdout.strip()
         env = dict(os.environ, GOFLAGS="-mod=mod", GOPROXY="off", GOTOOLCHAIN="local")
-        r = subprocess.run([go, "run", "."], cwd=os.path.join(ROOT, "oracle", "goprobe"), capture_output=True, text=True, timeout=120, env=env,
-                           input=open(os.path.join(ROOT, "tests", "golden", "hash_kats.json")).read())
+        with tempfile.TemporaryDirectory() as tmp:          # -mod=mod may write go.sum: run a copy, not the tree
+            probe = shutil.copytree(os.path.join(ROOT, "oracle", "goprobe"), os.path.join(tmp, "goprobe"))
+            r = subprocess.run([go, "run", "."], cwd=probe, capture_output=True, text=True, timeout=120, env=env,
+                               input=open(os.path.join(ROOT, "tests", "golden", "hash_kats.json")).read())
         if r.returncode != 0:
             return {"go": ver, "pinned": False, "why": "go run failed (module cache without fxamacker/cbor?): " + r.stderr.strip()[-200:]}
         res = json.loads(r.stdout)
@@ -430,6 +459,10 @@ def run_ours(args):
             b.record(stream)
         t_all1.record(stream)
         barrier()
+        if args.dump_outputs and mode == primary and rank == 0:
+            rows = dump_rows(Q)
+            sel = torch.from_numpy(rows).to(dev)
+            dump_outputs(args.dump_outputs, rows, d_scores.index_select(0, sel).cpu().numpy(), d_has.index_select(0, sel).cpu().numpy())
         launches = ixx.stats()["kernel_launches"] - launches0
         total_ms = max_ranks(t_all0.elapsed_time(t_all1))
         t_wait = time.time()
@@ -813,13 +846,17 @@ def emit(obj):
 
 
 def main():
+    sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (it may be read-only)
     quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,13 +3,13 @@
 (tests/e2e/redis_mock/e2e_test.go:109-244) tokenized with the reference's own checked-in tokenizer
 (tests/e2e/redis_mock/testdata/test-model/tokenizer.json, BERT uncased, add_special_tokens=False as in
 pkg/tokenization/tokenizer.go:411) by the HF `tokenizers` core -- the library the reference links.
-Run in the build container (needs /root/reference); the GPU box only reads the committed JSON."""
+Usage: python tests/golden/make_e2e_tokens.py REFERENCE_CHECKOUT; the tests only read the committed JSON."""
 import json
 import os
+import sys
 
 from tokenizers import Tokenizer
 
-REF = "/root/reference/tests/e2e/redis_mock/testdata/test-model/tokenizer.json"
 FULL = ("lorem ipsum dolor sit amet, consectetur adipiscing elit. Sed do eiusmod tempor incididunt ut labore et dolore magna aliqua. "
         "Ut enim ad minim veniam, quis nostrud exercitation ullamco laboris nisi ut aliquip ex ea commodo consequat.")
 MID = "lorem ipsum dolor sit amet, consectetur adipiscing elit. Sed do eiusmod tempor incididunt ut labore et dolore magna aliqua."
@@ -20,7 +20,7 @@ PROMPTS = {"full": FULL, "mid": MID, "short": SHORT, "miss": "What is the capita
 
 
 def main():
-    tok = Tokenizer.from_file(REF)
+    tok = Tokenizer.from_file(os.path.join(sys.argv[1], "tests", "e2e", "redis_mock", "testdata", "test-model", "tokenizer.json"))
     out = {"tokenizer": "tests/e2e/redis_mock/testdata/test-model/tokenizer.json (reference @ a378f5b3)", "block_size": 4, "prompts": {}}
     for name, p in PROMPTS.items():
         enc = tok.encode(p, add_special_tokens=False)

@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generates the committed golden fixtures in tests/golden/.
 
-Run from the repo root in the BUILD container (needs /root/reference for the
-reference's own fixture, python `cbor2` as the independent CBOR implementation):
+Run from the repo root with a checkout of the reference project (for its own fixture) and
+python `cbor2` (the independent CBOR implementation):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py REFERENCE_CHECKOUT
 
 Outputs
   hash_kats.json     request-key known answers.  The expected values are computed with
@@ -103,7 +103,7 @@ def hash_kats():
 
 
 def kv_event_base():
-    src = "/root/reference/tests/integration/testdata/kv_event_base.json"
+    src = os.path.join(sys.argv[1], "tests", "integration", "testdata", "kv_event_base.json")
     d = json.load(open(src))
     keys = chain(d["hash_seed"], d["token_ids"], d["block_size"])
     assert keys[:3] == [1232996234064703281, 4081027702767042585, 6770700869230650880] and keys[-1] == 4842047765409919357
